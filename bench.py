@@ -3,6 +3,7 @@
 
 Contract (see DESIGN.md §Measurement):
   python bench.py --gpus N --steps K --warmup W        one JSON line on stdout (rank 0)
+  python bench.py ... --dump-outputs DIR               also every linear's output of the last timed step, DIR/<linear>.npy
   python bench.py --impl reference ...                 the reference's OWN CPU code (baseline/_ref, unmodified) on host cores
 
 A "step" is ONE decode-token pass over every quantized linear of the model named in `config.workload`
@@ -149,8 +150,7 @@ def cpu_layer_sample(model, K, nbits, target_seconds, nthreads=0):
 
     from oracle import c_oracle
 
-    c_oracle.build()
-    threads = nthreads or c_oracle.num_threads()
+    threads = nthreads or c_oracle.num_threads()  # the library build() made: no rebuild here, the tree may be read-only
     rng = np.random.default_rng(0)
     lins = []
     for _, fin, fout in layer_linears(model):
@@ -357,6 +357,27 @@ def build_model(model, K, nbits, n_layers, device, rank, world, peer_comm=None):
             mods.append((m, local_groups * 8))
         layers.append(mods)
     return layers
+
+
+DUMP_LIMIT_BYTES = 64 * 2**20
+
+
+def dump_outputs(out_dir, model, ys):
+    """`--dump-outputs`: what one timed step returned to its caller, so that two builds can be compared output for output.
+    `ys` holds every linear's output of the step, layer after layer in layer_linears order; each linear is written as
+    `<out_dir>/<name>.npy`, float32 [layers, batch, out_features].  When the whole step exceeds DUMP_LIMIT_BYTES (only with
+    a large `--layers`), a fixed, evenly spaced subset of the layers is written instead."""
+    import numpy as np
+
+    names = [name for name, _, _ in layer_linears(model)]
+    per_layer = [ys[i:i + len(names)] for i in range(0, len(ys), len(names))]
+    layer_bytes = 4 * sum(y.numel() for y in per_layer[0])
+    keep = max(1, min(len(per_layer), DUMP_LIMIT_BYTES // layer_bytes))
+    idx = np.unique(np.linspace(0, len(per_layer) - 1, keep).round().astype(int))
+    os.makedirs(out_dir, exist_ok=True)
+    for j, name in enumerate(names):
+        arr = np.stack([per_layer[i][j].float().cpu().numpy() for i in idx])
+        np.save(os.path.join(out_dir, f"{name}.npy"), arr)
 
 
 def group_layers(layers, K, nbits, world):
@@ -656,16 +677,19 @@ def run_ours(args):
     if grouped:
         layers = group_layers(layers, K, nbits, world)
     in_sizes = sorted({n for mods in layers for _, n in mods})
-    x_dev = {n: torch.randn((1, n), dtype=torch.float16, device=device) for n in in_sizes}
+    gen_x = torch.Generator(device=device).manual_seed(99)
+    x_dev = {n: torch.randn((1, n), dtype=torch.float16, device=device, generator=gen_x) for n in in_sizes}
     x_host = {n: torch.randn((1, n), dtype=torch.float16).pin_memory() for n in in_sizes}
     outs = {}
 
     def step():
-        y = None
+        ys = []
         for mods in layers:
             for m, n in mods:
                 y = m(x_dev[n])
-        outs["y"] = y[-1] if isinstance(y, tuple) else y
+                ys.extend(y if isinstance(y, tuple) else (y,))
+        outs["all"] = ys  # every linear's output, in layer_linears order per layer
+        outs["y"] = ys[-1]
 
     # bind kernels / NCCL outside capture, count launches of one step
     step()
@@ -713,6 +737,8 @@ def run_ours(args):
     sampler = ClockSampler(local_rank) if rank == 0 else None
     ms_total = timed(run, args.steps)
     ms_step = ms_total / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, outs["all"])
 
     # ---- e2e: pinned-host activations in, last output out, every step ---------------------------------
     y_host = torch.empty_like(outs["y"], device="cpu").pin_memory()
@@ -988,7 +1014,13 @@ def main():
     ap.add_argument("--skip-reference-gpu", action="store_true", help="skip the reference CUDA kernels / generate legs")
     ap.add_argument("--watchdog-seconds", type=float, default=420.0,
                     help="N>1: leave with an error line if one phase (parity, build, timing, ...) takes longer than this (0: off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write every linear's output of the last timed step as DIR/<linear>.npy (float32, seeded inputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -44,3 +44,38 @@ def test_watchdog_ends_a_stuck_phase_and_respects_cancel():
     assert lines[:2] == ["survived", "disabled ok"] and "NOT REACHED" not in r.stdout
     err = json.loads(lines[-1])
     assert "stuck exchange" in err["error"] and err["rank"] == 0
+
+
+def test_dump_outputs_one_float32_file_per_linear(tmp_path):
+    import numpy as np
+    import torch
+
+    lins = bench.layer_linears("llama3-8b")
+    ys = [torch.full((1, fout), float(layer), dtype=torch.float16) for layer in range(3) for _, _, fout in lins]
+    bench.dump_outputs(str(tmp_path / "out"), "llama3-8b", ys)
+    assert sorted(os.listdir(tmp_path / "out")) == sorted(f"{name}.npy" for name, _, _ in lins)
+    for name, _, fout in lins:
+        a = np.load(tmp_path / "out" / f"{name}.npy")
+        assert a.dtype == np.float32 and a.shape == (3, 1, fout)
+        assert a[:, 0, 0].tolist() == [0.0, 1.0, 2.0]
+
+
+def test_dump_outputs_keeps_a_fixed_layer_subset_under_the_limit(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+
+    lins = bench.layer_linears("llama3-8b")
+    layer_bytes = 4 * sum(fout for _, _, fout in lins)
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 3 * layer_bytes)
+    ys = [torch.full((1, fout), float(layer), dtype=torch.float16) for layer in range(9) for _, _, fout in lins]
+    bench.dump_outputs(str(tmp_path), "llama3-8b", ys)
+    total = sum(os.path.getsize(tmp_path / f) for f in os.listdir(tmp_path))
+    assert total <= 3 * layer_bytes + 128 * len(lins)  # + the .npy headers
+    for name, _, _ in lins:
+        assert np.load(tmp_path / f"{name}.npy")[:, 0, 0].tolist() == [0.0, 4.0, 8.0]
+
+
+def test_steps_below_one_are_refused():
+    r = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=120)
+    assert r.returncode == 2 and "--steps" in r.stderr
