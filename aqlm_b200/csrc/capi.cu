@@ -612,15 +612,20 @@ struct GemmPlan {
 
 static GemmPlan gemm_plan(const aqlm_b200_weight_t* w, int64_t batch, const DeviceInfo* di, bool allow_split) {
   GemmPlan g;
-  const int K = w->num_codebooks, nbits = w->nbits_per_codebook;
+  const int K = w->num_codebooks, nbits = w->nbits_per_codebook, gs = w->in_group_size;
   const int cb = nbits <= 8 ? 1 : 2;
-  if (w->in_group_size != 8 || (nbits != 8 && nbits != 16)) return g;
+  const bool g16 = gs == 16;
+  if (nbits != 8 && nbits != 16) return g;
+  // in_group_size 16: the 1x16 scheme only; its 256-bit gathers need a 32-byte aligned codebook (any torch allocation is)
+  // No batch threshold: the tensor-core kernel beat the GEMV passes at every measured Llama-3-8B shape and batch, by
+  // 2.2-4.0x at 7 rows and 28-75x at 256 (profiles/r03/probe_gemm_g16_matmat_dequant.jsonl)
+  if (g16 && (K != 1 || nbits != 16 || (reinterpret_cast<uintptr_t>(w->codebooks) & 31) != 0)) return g;
   if (!(K == 1 || K == 2 || K == 4 || K == 8) || 8 * K * cb > kCodeTileBytes) return g;
   if (w->in_features % kGemmBlockK != 0) return g;
   if ((reinterpret_cast<uintptr_t>(w->codes) & 15) != 0) return g;
-  // TMA needs a 16-byte multiple as the global row stride of the code matrix (1x8: in_features % 128 == 0);
+  // TMA needs a 16-byte multiple as the global row stride of the code matrix (1x8 and 1x16 g16: in_features % 128 == 0);
   // other shapes take the GEMV fallback in aqlm_b200_matmat_dequant_ws
-  if (((size_t)(w->in_features / 8) * K * cb) % 16 != 0) return g;
+  if (((size_t)(w->in_features / gs) * K * cb) % 16 != 0) return g;
   if (tun().disable_tcgen05) return g;
   g.total_kblocks = (int)(w->in_features / kGemmBlockK);
   if (batch <= 256) {
@@ -635,6 +640,8 @@ static GemmPlan gemm_plan(const aqlm_b200_weight_t* w, int64_t batch, const Devi
   // A in tensor memory: measured 1x16 61.7 -> 55.1 us, 2x8 69.3 -> 49.2 us (4096->14336/11008, bs=256); 8x8 no gain
   g.atmem = (tun().gemm_atmem < 0 ? (K <= 2) : tun().gemm_atmem != 0) && !(tun().gemm_debug & 1);
   g.v2 = g.atmem || ((tun().gemm_v2 < 0 ? (K >= 4 ? 1 : 0) : tun().gemm_v2) != 0 && !(tun().gemm_debug & 1));
+  // in_group_size 16 is built in the V2 + A-in-TMEM form only: switches that force another form leave it to the GEMV passes
+  if (g16 && (!g.atmem || tun().gemm_v2 == 0)) return g;
   const size_t budget = (size_t)di->max_smem_optin;
   // At most 3 stages: shared memory taken here is L1 taken from the codebook gathers (outstanding misses need L1
   // lines); measured at N=256: 4 stages 335 TFLOP/s, 3 stages 484-503, 2 stages 470 (profiles/r01/gemm_experiments.md)
@@ -662,9 +669,11 @@ static GemmPlan gemm_plan(const aqlm_b200_weight_t* w, int64_t batch, const Devi
   //   per CTA: its k-blocks + a fixed cost (launch ramp, TMEM alloc, pipeline fill, epilogue: ~5 us measured);
   //   per launch: waves x CTA time + split-K fix-up traffic (partials written and read once through L2).
   // The gather rate is the measured per-SM rate of random 16-byte codebook reads (profiles/: ~0.85/clk from L2 for the
-  // 1 MiB 1x16 codebook; 256-entry codebooks are L1-resident and gather faster).
+  // 1 MiB 1x16 codebook; 256-entry codebooks are L1-resident and gather faster).  in_group_size 16 issues 4 gathers per
+  // row per k-block, each one 32-byte request; the GEMM's rate of those is not measured, so the 16-byte rate stands in.
   const double clk = 1.9e9;
   const double gather_per_clk = (nbits == 16 ? 0.85 : 1.6) * (g.atmem ? 1.0 : 0.7);  // SS form: smaller L1 -> slower gathers
+  const double gathers_per_row = (double)(kGemmBlockK / gs) * K;
   const double t_mma = 2.0 * g.n_tile;                                                 // 4 x (128 x N x 16) at 4096 MAC/clk
   int best_tm = kGemmBlockM, best_ks = 1;
   double best = 1e30;
@@ -675,7 +684,7 @@ static GemmPlan gemm_plan(const aqlm_b200_weight_t* w, int64_t batch, const Devi
     if (tiles > kGemmMaxTiles) continue;
     // CTA pairs multicast the X tile: keep the number of M tiles even (full-height tiles stay as the fallback)
     if (want_pairs && tm != kGemmBlockM && (((w->out_features + tm - 1) / tm) & 1)) continue;
-    const double t_gather = tm * 8.0 * K / gather_per_clk;
+    const double t_gather = tm * gathers_per_row / gather_per_clk;
     const double t_smem = (g.atmem ? 0.0 : (128.0 + tm) * 128.0 / 128.0) + 2.0 * g.n_tile;  // bytes / (128 B/clk)
     const double t_kb = (t_gather > t_mma ? (t_gather > t_smem ? t_gather : t_smem) : (t_mma > t_smem ? t_mma : t_smem)) + 60.0;
     for (int c = 1; c <= max_ks; ++c) {
@@ -713,9 +722,10 @@ static GemmPlan gemm_plan(const aqlm_b200_weight_t* w, int64_t batch, const Devi
   return g;
 }
 
-template <typename T, int K, int CB>
+template <typename T, int K, int CB, int GS = 8>
 static int launch_gemm(const aqlm_b200_weight_t* w, const void* input, void* output, int64_t batch, const GemmPlan& g,
                        void* workspace, cudaStream_t st) {
+  const size_t row_bytes = (size_t)(w->in_features / GS) * K * CB;
   const DeviceInfo* di = device_info();
   if (!di) return AQLM_B200_ERR_CUDA;
   tmap_encode_fn enc = get_tmap_encode();
@@ -733,7 +743,6 @@ static int launch_gemm(const aqlm_b200_weight_t* w, const void* input, void* out
     if (r != CUDA_SUCCESS) return fail(AQLM_B200_ERR_CUDA, "cuTensorMapEncodeTiled(x) failed: %d", (int)r);
   }
   {
-    const size_t row_bytes = (size_t)(w->in_features / 8) * K * CB;
     cuuint64_t dims[2] = {(cuuint64_t)row_bytes, (cuuint64_t)w->out_features};
     cuuint64_t strides[1] = {(cuuint64_t)row_bytes};
     cuuint32_t box[2] = {(cuuint32_t)kCodeTileBytes, (cuuint32_t)g.tile_m};
@@ -764,12 +773,18 @@ static int launch_gemm(const aqlm_b200_weight_t* w, const void* input, void* out
   p.debug = tun().gemm_debug;
   p.gather_mode = tun().gemm_gather_mode >= 0 ? tun().gemm_gather_mode : (w->nbits_per_codebook > 8 ? 1 : 0);
   p.codes = w->codes;
-  p.row_bytes = (long long)(w->in_features / 8) * K * CB;
+  p.row_bytes = (long long)row_bytes;
   const size_t smem = gemm_smem_layout(g.stages, g.n_tile, g.atmem).total;
   const bool v2 = g.v2 && g.stages <= 4;
   const bool atmem = g.atmem && v2;
-  auto kernel = atmem ? gemm_dequant_kernel<T, K, CB, true, true>
-                      : (v2 ? gemm_dequant_kernel<T, K, CB, true, false> : gemm_dequant_kernel<T, K, CB, false, false>);
+  decltype(&gemm_dequant_kernel<T, K, CB, true, true>) kernel;
+  if constexpr (GS == 16) {
+    if (!atmem) return fail(AQLM_B200_ERR_UNSUPPORTED, "in_group_size 16 GEMM is built in the V2 + A-in-TMEM form only");
+    kernel = gemm_dequant_kernel<T, K, CB, true, true, 16>;
+  } else {
+    kernel = atmem ? gemm_dequant_kernel<T, K, CB, true, true>
+                   : (v2 ? gemm_dequant_kernel<T, K, CB, true, false> : gemm_dequant_kernel<T, K, CB, false, false>);
+  }
   static SmemMarks marks[3];
   if (int rc = ensure_smem(kernel, smem, marks[atmem ? 2 : (v2 ? 1 : 0)], di)) return rc;
   cudaLaunchConfig_t cfg = {};
@@ -795,6 +810,7 @@ template <typename T>
 static int gemm_typed(const aqlm_b200_weight_t* w, const void* input, void* output, int64_t batch, const GemmPlan& g,
                       void* workspace, cudaStream_t st) {
   const int K = w->num_codebooks, cb = w->nbits_per_codebook <= 8 ? 1 : 2;
+  if (w->in_group_size == 16) return launch_gemm<T, 1, 2, 16>(w, input, output, batch, g, workspace, st);  // gemm_plan: 1x16 only
   if (cb == 2 && K == 1) return launch_gemm<T, 1, 2>(w, input, output, batch, g, workspace, st);
   if (cb == 2 && K == 2) return launch_gemm<T, 2, 2>(w, input, output, batch, g, workspace, st);
   if (cb == 2 && K == 4) return launch_gemm<T, 4, 2>(w, input, output, batch, g, workspace, st);
@@ -814,13 +830,15 @@ struct GemmTPlan {
 
 static GemmTPlan gemm_t_plan(const aqlm_b200_weight_t* w, int64_t batch, const DeviceInfo* di, bool allow_split) {
   GemmTPlan g;
-  const int K = w->num_codebooks, nbits = w->nbits_per_codebook;
+  const int K = w->num_codebooks, nbits = w->nbits_per_codebook, gs = w->in_group_size;
   const int cb = nbits <= 8 ? 1 : 2;
-  if (w->in_group_size != 8 || (nbits != 8 && nbits != 16)) return g;
+  if (nbits != 8 && nbits != 16) return g;
+  // in_group_size 16: 1x16 only, 256-bit gathers from a 32-byte aligned codebook
+  if (gs == 16 && (K != 1 || nbits != 16 || (reinterpret_cast<uintptr_t>(w->codebooks) & 31) != 0)) return g;
   if (!(K == 1 || K == 2 || K == 4 || K == 8) || 16 * K * cb > 256) return g;
   if (w->out_features % 8 != 0) return g;  // TMA row stride of grad_out
   if ((reinterpret_cast<uintptr_t>(w->codes) & 15) != 0) return g;
-  if (((size_t)(w->in_features / 8) * K * cb) % 16 != 0) return g;
+  if (((size_t)(w->in_features / gs) * K * cb) % 16 != 0) return g;  // 1x8 and 1x16 g16: in_features % 128 == 0
   if (tun().disable_tcgen05) return g;
   g.total_kblocks = (int)((w->out_features + kGemmBlockK - 1) / kGemmBlockK);
   g.m_tiles = (int)((w->in_features + kGemmBlockM - 1) / kGemmBlockM);
@@ -831,7 +849,7 @@ static GemmTPlan gemm_t_plan(const aqlm_b200_weight_t* w, int64_t batch, const D
     g.n_tile = 256;
     g.n_tiles = (int)((batch + 255) / 256);
   }
-  const int ctile_row_bytes = 16 * K * cb;
+  const int ctile_row_bytes = (kGemmBlockM / gs) * K * cb;
   const size_t budget = (size_t)di->max_smem_optin;
   int S = 3;
   while (S > 2 && gemm_t_smem_layout(S, g.n_tile, ctile_row_bytes).total > budget) --S;
@@ -844,7 +862,8 @@ static GemmTPlan gemm_t_plan(const aqlm_b200_weight_t* w, int64_t batch, const D
     // same cost model as the forward plan: a k-block costs max(gathers, tensor pipe, smem traffic), every wave pays a
     // fixed ~5 us, split-K partials go through L2 once each way
     const double clk = 1.9e9;
-    const double t_gather = 1024.0 * K / ((nbits == 16 ? 0.85 : 1.6) * 0.7);
+    // (64 out rows x 128 / in_group_size gathers; the 32-byte gathers of in_group_size 16 are costed at the 16-byte rate)
+    const double t_gather = 64.0 * (kGemmBlockM / gs) * K / ((nbits == 16 ? 0.85 : 1.6) * 0.7);
     const double t_smem = 256.0 + 2.0 * g.n_tile, t_mma = 2.0 * g.n_tile;
     const double t_kb = (t_gather > t_smem ? (t_gather > t_mma ? t_gather : t_mma) : (t_smem > t_mma ? t_smem : t_mma)) + 60.0;
     const double tiles = (double)g.m_tiles * g.n_tiles;
@@ -872,14 +891,14 @@ static GemmTPlan gemm_t_plan(const aqlm_b200_weight_t* w, int64_t batch, const D
   return g;
 }
 
-template <typename T, int K, int CB>
+template <typename T, int K, int CB, int GS = 8>
 static int launch_gemm_t(const aqlm_b200_weight_t* w, const void* grad_output, void* grad_input, int64_t batch,
                          const GemmTPlan& g, void* workspace, cudaStream_t st) {
   const DeviceInfo* di = device_info();
   if (!di) return AQLM_B200_ERR_CUDA;
   tmap_encode_fn enc = get_tmap_encode();
   if (!enc) return fail(AQLM_B200_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-  constexpr int GBT = 16 * K * CB;
+  constexpr int GBT = (kGemmBlockM / GS) * K * CB;  // code bytes per out row per 128-in-feature tile (TMA box, >= 16)
   ensure_driver_context();
   CUtensorMap tg, tc;
   {
@@ -893,7 +912,7 @@ static int launch_gemm_t(const aqlm_b200_weight_t* w, const void* grad_output, v
     if (r != CUDA_SUCCESS) return fail(AQLM_B200_ERR_CUDA, "cuTensorMapEncodeTiled(grad_output) failed: %d", (int)r);
   }
   {
-    const size_t row_bytes = (size_t)(w->in_features / 8) * K * CB;
+    const size_t row_bytes = (size_t)(w->in_features / GS) * K * CB;
     cuuint64_t dims[2] = {(cuuint64_t)row_bytes, (cuuint64_t)w->out_features};
     cuuint64_t strides[1] = {(cuuint64_t)row_bytes};
     cuuint32_t box[2] = {(cuuint32_t)GBT, (cuuint32_t)kGemmTCtileRows};
@@ -919,7 +938,7 @@ static int launch_gemm_t(const aqlm_b200_weight_t* w, const void* grad_output, v
   p.stages = g.stages;
   p.gather_mode = tun().gemm_gather_mode >= 0 ? tun().gemm_gather_mode : (w->nbits_per_codebook > 8 ? 1 : 0);
   const size_t smem = gemm_t_smem_layout(g.stages, g.n_tile, GBT).total;
-  auto kernel = gemm_dequant_t_kernel<T, K, CB>;
+  auto kernel = gemm_dequant_t_kernel<T, K, CB, GS>;
   static SmemMarks marks;
   if (int rc = ensure_smem(kernel, smem, marks, di)) return rc;
   cudaLaunchConfig_t cfg = {};
@@ -941,6 +960,7 @@ template <typename T>
 static int gemm_t_typed(const aqlm_b200_weight_t* w, const void* grad_output, void* grad_input, int64_t batch,
                         const GemmTPlan& g, void* workspace, cudaStream_t st) {
   const int K = w->num_codebooks, cb = w->nbits_per_codebook <= 8 ? 1 : 2;
+  if (w->in_group_size == 16) return launch_gemm_t<T, 1, 2, 16>(w, grad_output, grad_input, batch, g, workspace, st);  // 1x16 only
   if (cb == 2 && K == 1) return launch_gemm_t<T, 1, 2>(w, grad_output, grad_input, batch, g, workspace, st);
   if (cb == 2 && K == 2) return launch_gemm_t<T, 2, 2>(w, grad_output, grad_input, batch, g, workspace, st);
   if (cb == 2 && K == 4) return launch_gemm_t<T, 4, 2>(w, grad_output, grad_input, batch, g, workspace, st);
@@ -1128,7 +1148,8 @@ int aqlm_b200_matmat_dequant_ws(const aqlm_b200_weight_t* w, const void* input, 
   GemmPlan g = gemm_plan(w, batch, di, workspace != nullptr);
   if (g.ok && g.ksplit > 1 && workspace_bytes < g.counters_bytes + g.partials_bytes) g = gemm_plan(w, batch, di, false);
   if (!g.ok || (reinterpret_cast<uintptr_t>(input) & 15) != 0) {
-    // shapes the tensor-core kernel does not cover (in_group 16, in_features % 64 != 0, odd KxN):
+    // shapes the tensor-core kernel does not cover (in_features % 64 != 0, code rows not a 16-byte multiple, odd KxN,
+    // in_group 16 other than 1x16):
     // batch passes of 8 rows through the fused gather+dequant+dot kernel
     return aqlm_b200_matmat_ex(w, input, output, batch, 0, stream);
   }
@@ -1176,8 +1197,8 @@ int aqlm_b200_matmat_dequant_transposed(const aqlm_b200_weight_t* w, const void*
   if (g.ok && g.ksplit > 1 && workspace_bytes < g.counters_bytes + g.partials_bytes) g = gemm_t_plan(w, batch, di, false);
   if (!g.ok)
     return fail(AQLM_B200_ERR_UNSUPPORTED,
-                "matmat_dequant_transposed: the fused kernel covers in_group_size 8, 8/16-bit codes, 1/2/4/8 codebooks, "
-                "16-byte aligned code rows and out_features %% 8 == 0");
+                "matmat_dequant_transposed: the fused kernel covers in_group_size 8 (8/16-bit codes, 1/2/4/8 codebooks) and "
+                "in_group_size 16 (1x16, 32-byte aligned codebook), 16-byte aligned code rows and out_features %% 8 == 0");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (w->dtype == AQLM_B200_F16) return gemm_t_typed<__half>(w, grad_output, grad_input, batch, g, workspace, st);
   return gemm_t_typed<__nv_bfloat16>(w, grad_output, grad_input, batch, g, workspace, st);

@@ -177,19 +177,22 @@ __host__ __device__ inline GemmSmem gemm_smem_layout(int stages, int n_tile, boo
   return L;
 }
 
-// K = codebooks per group, CODE_BYTES = 1|2 ; in_group_size == 8.
-// bytes of codes per row per 64-wide k-block: GB = 8 groups * K * CODE_BYTES
+// K = codebooks per group, CODE_BYTES = 1|2, GS = in_group_size (8, or 16 for 1x16 in the V2 + ATMEM form only).
+// bytes of codes per row per 64-wide k-block: GB = (64 / GS) groups * K * CODE_BYTES
+// GS = 16: a codebook entry is 16 halves = one 32-byte sector, fetched as ONE 256-bit request (ld_gather_v8), so a
+// k-block costs 4 gather requests per row instead of 8; the entry fills 8 of the row's 32 TMEM columns unchanged.
 // ATMEM (needs the V2 producer mapping, thread <-> row): the dequantized A tile is written to TENSOR MEMORY with tcgen05.st
 // and the MMA takes A from TMEM.  Shared memory then carries only the X stages (and the code tiles): per k-block the
 // shared-memory traffic drops from 96 KB (A write + A read + X write + X read at N=256) to 64 KB -- at 128 B/clk that was
 // 768 clk against 512 clk of MMA, i.e. the SS form was shared-memory bound before any gather -- and the L1 the gathers
 // run against grows by the 48 KB the A stages took.
-template <typename T, int K, int CODE_BYTES, bool V2, bool ATMEM = false>
+template <typename T, int K, int CODE_BYTES, bool V2, bool ATMEM = false, int GS = 8>
 __global__ void __launch_bounds__(V2 ? kGemmThreadsV2 : kGemmThreads, 1)
 gemm_dequant_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_codes, const GemmParams p) {
   static_assert(!ATMEM || V2, "A-in-TMEM needs the thread <-> row producer mapping");
+  static_assert(GS == 8 || (GS == 16 && K == 1 && CODE_BYTES == 2 && V2 && ATMEM), "in_group_size 16: 1x16, V2 + ATMEM only");
   constexpr int NTHREADS = V2 ? kGemmThreadsV2 : kGemmThreads;
-  constexpr int GB = 8 * K * CODE_BYTES;             // code bytes per row per k-block
+  constexpr int GB = (kGemmBlockK / GS) * K * CODE_BYTES;  // code bytes per row per k-block
   constexpr int KB_PER_CTILE = kCodeTileBytes / GB;  // k-blocks covered by one code tile
   static_assert(KB_PER_CTILE >= 1, "scheme too wide for the code tile");
   extern __shared__ uint8_t smem_dyn[];
@@ -380,7 +383,7 @@ gemm_dequant_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_con
                 const uint4 v = *reinterpret_cast<const uint4*>(crow + (chunk << 4));
                 cw[q * 4 + 0] = v.x; cw[q * 4 + 1] = v.y; cw[q * 4 + 2] = v.z; cw[q * 4 + 3] = v.w;
               }
-            } else {  // GB == 8 (1x8)
+            } else {  // GB == 8 (1x8; 1x16 with GS = 16)
               const int lb = st_in * GB;
               const int chunk = (lb >> 4) ^ (row & 7);
               const uint2 v = *reinterpret_cast<const uint2*>(crow + (chunk << 4) + (lb & 15));
@@ -392,7 +395,20 @@ gemm_dequant_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_con
             else return (cw[idx >> 2] >> ((idx & 3) * 8)) & 0xffu;
           };
           auto gather_all = [&](const uint32_t (&cw)[CWN], uint4 (&wv)[8][INREG ? K : 1]) {
-            if constexpr (INREG) {
+            if constexpr (GS == 16) {
+              // group q = 16 halves = TMEM columns [8q, 8q+8): one 256-bit gather into wv[2q] (lo) and wv[2q+1] (hi)
+              if (active && !(p.debug & 8)) {
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                  const uint4* gp = gcb + 2 * (size_t)code_at(cw, q);
+                  if (p.gather_mode == 1) ld_gather_v8<1>(gp, wv[2 * q][0], wv[2 * q + 1][0]);
+                  else ld_gather_v8<0>(gp, wv[2 * q][0], wv[2 * q + 1][0]);
+                }
+              } else {
+#pragma unroll
+                for (int e = 0; e < 8; ++e) wv[e][0] = make_uint4(0u, 0u, 0u, 0u);
+              }
+            } else if constexpr (INREG) {
               if (active && !(p.debug & 8)) {
 #pragma unroll
                 for (int e = 0; e < 8; ++e)

@@ -12,7 +12,7 @@
 //       64 x 8 element atoms, instruction descriptor a_major = 1), so a gather still lands with ONE 16-byte store;
 //       the per-row scale is applied to the vector before it is written (fp32 multiply, one rounding);
 //   B = grad_out tile [N x 64 out columns], K-major, TMA-loaded with 128B swizzle (OOB rows/columns zero-filled);
-//   code tiles: TMA boxes of 256 out rows x (16 groups * K codes) bytes, un-swizzled.
+//   code tiles: TMA boxes of 256 out rows x (128 / in_group_size groups * K codes) bytes, un-swizzled.
 // Grid = (in/128 tiles, K splits over the out rows, N tiles); split partials and the deterministic last-CTA fix-up are
 // the forward kernel's.
 #pragma once
@@ -71,11 +71,14 @@ __host__ __device__ inline GemmTSmem gemm_t_smem_layout(int stages, int n_tile, 
   return L;
 }
 
-template <typename T, int K, int CODE_BYTES>
+// GS = in_group_size.  GS = 16 (1x16 only): a thread's 16 in-features are ONE codebook entry of 32 bytes, fetched as one
+// 256-bit request and stored as the same two 16-byte chunks along M that two 8-wide groups fill.
+template <typename T, int K, int CODE_BYTES, int GS = 8>
 __global__ void __launch_bounds__(kGemmTThreads, 1)
 gemm_dequant_t_kernel(const __grid_constant__ CUtensorMap tmap_g, const __grid_constant__ CUtensorMap tmap_codes, const GemmTParams p) {
-  constexpr int GBT = 16 * K * CODE_BYTES;  // code bytes per out row per tile (16 groups = 128 in-features)
-  constexpr int CB2 = 2 * K * CODE_BYTES;   // code bytes of one thread's 2 adjacent groups
+  static_assert(GS == 8 || (GS == 16 && K == 1 && CODE_BYTES == 2), "in_group_size 16: 1x16 only");
+  constexpr int GBT = (kGemmBlockM / GS) * K * CODE_BYTES;  // code bytes per out row per tile (128 in-features)
+  constexpr int CB2 = GBT / 8;                              // code bytes of one thread's 16 in-features
   constexpr int CW = (CB2 + 3) / 4;
   constexpr int D = (K == 1) ? 4 : (K == 2 ? 2 : 1);  // k-blocks of gathers held in registers ahead of the writes
   constexpr int KB_PER_CTILE = kGemmTCtileRows / kGemmBlockK;
@@ -178,7 +181,8 @@ gemm_dequant_t_kernel(const __grid_constant__ CUtensorMap tmap_g, const __grid_c
       if (elect_one()) umma_commit(tfull_bar);
       __syncwarp();
     } else if (warp >= 4) {
-      // ===== dequant producers: 512 threads, thread -> (out row kk of the k-block, 2 adjacent in-groups) =====
+      // ===== dequant producers: 512 threads, thread -> (out row kk of the k-block, 16 consecutive in-features: 2 adjacent
+      //       groups of 8, or 1 group of 16) =====
       const int pt = threadIdx.x - 128;
       const int kk = pt >> 3, gp = pt & 7;  // kk: 0..63, gp: group pair 0..7 -> groups 2gp, 2gp+1 (of 16)
       const uint4* gcb = reinterpret_cast<const uint4*>(p.codebooks);
@@ -204,17 +208,23 @@ gemm_dequant_t_kernel(const __grid_constant__ CUtensorMap tmap_g, const __grid_c
         } else {
           cw[0] = *reinterpret_cast<const uint16_t*>(src);
         }
+        if constexpr (GS == 16) {
+          const uint4* gq = gcb + 2 * (size_t)(cw[0] & 0xffffu);
+          if (p.gather_mode == 1) ld_gather_v8<1>(gq, wv[0][0], wv[1][0]);
+          else ld_gather_v8<0>(gq, wv[0][0], wv[1][0]);
+        } else {
 #pragma unroll
-        for (int e = 0; e < 2; ++e) {
+          for (int e = 0; e < 2; ++e) {
 #pragma unroll
-          for (int k = 0; k < K; ++k) {
-            const int idx = e * K + k;
-            uint32_t code;
-            if constexpr (CODE_BYTES == 2) code = (cw[idx >> 1] >> ((idx & 1) * 16)) & 0xffffu;
-            else code = (cw[idx >> 2] >> ((idx & 3) * 8)) & 0xffu;
-            const uint4* gq = gcb + (((size_t)k << p.nbits) + code);
-            if (p.gather_mode == 1) wv[e][k] = ld_gather_v4<1>(gq);
-            else wv[e][k] = ld_gather_v4<0>(gq);
+            for (int k = 0; k < K; ++k) {
+              const int idx = e * K + k;
+              uint32_t code;
+              if constexpr (CODE_BYTES == 2) code = (cw[idx >> 1] >> ((idx & 1) * 16)) & 0xffffu;
+              else code = (cw[idx >> 2] >> ((idx & 3) * 8)) & 0xffu;
+              const uint4* gq = gcb + (((size_t)k << p.nbits) + code);
+              if (p.gather_mode == 1) wv[e][k] = ld_gather_v4<1>(gq);
+              else wv[e][k] = ld_gather_v4<0>(gq);
+            }
           }
         }
         if (st_in == KB_PER_CTILE - 1 || i == nkb - 1) {  // after the gathers were issued: the code reads have completed

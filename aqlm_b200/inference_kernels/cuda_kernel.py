@@ -253,8 +253,9 @@ def matmat_dequant_transposed(input, codes, codebooks, scales, bias=None) -> tor
     called.  The reference's 2x8/1x8 variants forget the scaled input (cuda_kernel.cpp:497,518,662,683); not reproduced.
     `bias` is the forward bias [out]; it has no place in grad_input (the reference passes it to F::linear,
     cuda_kernel.cpp:348-353, which only type-checks when in == out) and is ignored.
-    Layouts the fused kernel does not cover (in_group_size 16, odd codebook counts) fall back to our dequant kernel +
-    a dense matmul, as the reference does for every scheme.
+    The fused kernel covers in_group_size 8 and 1x16 with in_group_size 16 (in_features % 128 == 0).  Layouts it does
+    not cover (odd codebook counts, in_group_size 16 with several codebooks or 8-bit codes, ragged code rows) fall back
+    to our dequant kernel + a dense matmul, as the reference does for every scheme.
     """
     device = _require_cuda(input, codes, codebooks, scales)
     _dtype_code(input)

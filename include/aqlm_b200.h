@@ -95,7 +95,8 @@ int aqlm_b200_matmat_grouped(const aqlm_b200_weight_t* w, const int64_t* seg_row
 
 /* Fused dequant + tensor-core GEMM for large batch: W never goes to HBM.  Replaces
  * code{1x16,2x8,1x8}_matmat_dequant (cuda_kernel.cpp:249-301, 450-484, 615-649: Dequant kernel ->
- * full W in HBM -> cuBLAS F::linear -> epilogue). */
+ * full W in HBM -> cuBLAS F::linear -> epilogue).  Tensor-core kernel for in_group_size 8 and for 1x16 with
+ * in_group_size 16 (in_features % 128 == 0); other layouts run as passes of up to 8 rows through the fused GEMV. */
 int aqlm_b200_matmat_dequant(const aqlm_b200_weight_t* w, const void* input, void* output, int64_t batch, void* stream);
 /* Same with a caller-owned workspace, which lets the kernel split the K dimension across otherwise idle SMs
  * (the reduction is deterministic).  The first aqlm_b200_matmat_dequant_workspace_bytes() bytes... the whole
@@ -114,7 +115,9 @@ int aqlm_b200_dequant(const aqlm_b200_weight_t* w, void* weight_out, int apply_s
  * GEMM is involved.  Replaces code*_matmat_dequant_transposed (cuda_kernel.cpp:303-354, 486-519, 651-684: Dequant
  * kernel -> full W in HBM -> cuBLAS), with the 2x8/1x8 unscaled-input defect (cuda_kernel.cpp:497,518,662,683) NOT
  * reproduced.  The optional workspace (same zero-init contract as aqlm_b200_matmat_dequant_ws) enables split-K over the
- * out rows.  Returns AQLM_B200_ERR_UNSUPPORTED for layouts the fused kernel does not cover (in_group_size 16, ...). */
+ * out rows.  Covers in_group_size 8 (8/16-bit codes, 1/2/4/8 codebooks) and in_group_size 16 for 1x16 with
+ * in_features % 128 == 0; returns AQLM_B200_ERR_UNSUPPORTED for layouts the fused kernel does not cover (Kx8 or 2+
+ * codebooks with in_group_size 16, code rows that are not a 16-byte multiple, out_features % 8 != 0, ...). */
 size_t aqlm_b200_matmat_dequant_transposed_workspace_bytes(const aqlm_b200_weight_t* w, int64_t batch);
 int aqlm_b200_matmat_dequant_transposed(const aqlm_b200_weight_t* w, const void* grad_output, void* grad_input,
                                         int64_t batch, void* workspace, size_t workspace_bytes, void* stream);

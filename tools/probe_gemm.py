@@ -1,10 +1,14 @@
 """GEMM experiment probe: for each (shape, batch) and each environment setting, check the fused dequant + tcgen05 GEMM
 against the C oracle (row sample) and time it (CUDA-graph replay over rotating weight copies, CUDA events).
     python tools/probe_gemm.py [--shapes 4096x14336,4096x4096] [--batches 256] [--settings "A=1,B=2;A=0"] [--scheme 1x16]
-Each setting is a ';'-separated list of comma-separated ENV=VALUE pairs (AQLM_B200_ prefix added)."""
+                               [--in-group 16]
+Each setting is a ';'-separated list of comma-separated ENV=VALUE pairs (AQLM_B200_ prefix added); the settings of one
+(shape, batch) run back to back, so e.g. --settings "DISABLE_TCGEN05=1;" alternates the GEMV passes and the tensor-core
+path.  The first line records the device (name, power limit, SM clocks) the numbers were taken on."""
 import argparse
 import json
 import os
+import subprocess
 import sys
 
 import torch
@@ -15,7 +19,7 @@ sys.path.insert(0, os.path.join(REPO, "tests"))
 from aqlm_b200 import _cabi  # noqa: E402
 from aqlm_b200.inference_kernels import cuda_kernel  # noqa: E402
 
-KEYS = ["PDL", "GEMM_A_STAGES", "GEMM_GROUPS", "GEMM_ATMEM", "GEMM_TILE_M", "GEMM_KSPLIT", "GEMM_STAGES", "GEMM_V2", "GEMM_GATHER_MODE", "GEMM_DEBUG", "GEMM_CLUSTER"]
+KEYS = ["DISABLE_TCGEN05", "PDL", "GEMM_A_STAGES", "GEMM_GROUPS", "GEMM_ATMEM", "GEMM_TILE_M", "GEMM_KSPLIT", "GEMM_STAGES", "GEMM_V2", "GEMM_GATHER_MODE", "GEMM_DEBUG", "GEMM_CLUSTER"]
 
 
 def timed(fns, iters=10):
@@ -45,6 +49,7 @@ def main():
     ap.add_argument("--shapes", default="4096x14336,4096x4096,14336x4096")
     ap.add_argument("--batches", default="256")
     ap.add_argument("--scheme", default="1x16")
+    ap.add_argument("--in-group", type=int, default=8, choices=[8, 16])
     ap.add_argument("--dtype", default="f16")
     ap.add_argument("--op", default="matmat_dequant", choices=["matmat_dequant", "matmat_dequant_transposed"])
     ap.add_argument("--settings", default="")
@@ -54,11 +59,20 @@ def main():
     dt = torch.float16 if args.dtype == "f16" else torch.bfloat16
     settings = [dict(kv.split("=") for kv in st.split(",") if kv) for st in args.settings.split(";")] if args.settings else [{}]
     op = getattr(cuda_kernel, args.op)
+    g = args.in_group
+    dev = dict(device=torch.cuda.get_device_name(0))
+    try:
+        dev["nvidia_smi"] = subprocess.run(
+            ["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit,clocks.sm,clocks.max.sm", "--format=csv,noheader"],
+            capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError) as e:
+        dev["nvidia_smi"] = f"unavailable: {e}"
+    print(json.dumps(dev), flush=True)
     for shape in args.shapes.split(","):
         fin, fout = (int(v) for v in shape.split("x"))
         for bs in (int(b) for b in args.batches.split(",")):
-            t = gpu_case(fin, fout, K, nbits, bs, dtype=dt, seed=fin + fout + bs)
-            cbytes = fout * (fin // 8) * K * (2 if nbits > 8 else 1)
+            t = gpu_case(fin, fout, K, nbits, bs, dtype=dt, seed=fin + fout + bs, g=g)
+            cbytes = fout * (fin // g) * K * (2 if nbits > 8 else 1)
             copies = max(2, min(24, 300 * 2**20 // cbytes))
             lo, hi = (-128, 128) if nbits <= 8 else (-32768, 32768)
             ws = [(t["codes"], t["codebooks"], t["scales"])] + [
@@ -72,10 +86,12 @@ def main():
                 for k, v in st.items():
                     os.environ["AQLM_B200_" + k] = v
                 _cabi.reload_tunables()
-                row = dict(op=args.op, scheme=args.scheme, dtype=args.dtype, shape=shape, batch=bs, setting=st)
+                row = dict(op=args.op, scheme=args.scheme, in_group=g, dtype=args.dtype, shape=shape, batch=bs, setting=st)
                 try:
+                    c0 = _cabi.launch_count()
                     y = op(x, t["codes"], t["codebooks"], t["scales"], None)
                     torch.cuda.synchronize()
+                    row["launches"] = _cabi.launch_count() - c0
                     if not args.no_check:
                         if transposed:
                             W = cuda_kernel.dequant(t["codes"], t["codebooks"], t["scales"]).float()
